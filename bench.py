@@ -18,6 +18,8 @@ the only exchange the path has.  No PyTorch kernel runs inside a step.
              C4 (n=16 commit-vote quorum stream, 262,144 signatures, sharded by instance over the ranks), C5 (mixed curves)
 
 `--impl reference` times the CPU implementation alone (the reference arm).
+`--dump-outputs DIR` writes the verdicts of the last timed step as float32 .npy files; the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -139,6 +141,8 @@ def run_reference(args, rank, world):
     for _ in range(args.steps):
         t, ok = oracle.bench_verify(oracle.P256, b["r"], b["s"], keys, b["key_idx"], b["digest"], nthreads=cores)
         total += t
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"verdicts": ok})
     value = BATCH * args.steps / total
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "verifies/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -158,6 +162,15 @@ def pack_bits(ok):
     return np.packbits(ok.astype(np.uint8), bitorder="little").view(np.uint32)
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy in float32 (verdicts are 0/1, so the conversion is exact): what the timed
+    path returned in its last step, for comparing two builds output for output on the same seeded inputs."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -166,7 +179,11 @@ def main():
     ap.add_argument("--impl", default="sbv", choices=["sbv", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the verdicts of the last one as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -302,6 +319,13 @@ def main():
             raise SystemExit("bench: pipelined verdicts differ from the oracle")
         if world > 1 and not np.array_equal(d_masks[k].cpu().numpy(), want_mask_all):
             raise SystemExit("bench: gathered verdict mask differs from the packed oracle verdicts of all ranks")
+    if args.dump_outputs and rank == 0:
+        # the lane of the last timed step; the registered-key leg below reuses these buffers
+        last = (args.warmup + args.steps - 1) % N_LANES
+        outputs = {"verdicts": d_oks[last].cpu().numpy()}
+        if world > 1:   # the gathered mask every rank receives, one 0/1 entry per item of all ranks
+            outputs["gathered_verdicts"] = np.unpackbits(d_masks[last].cpu().numpy().view(np.uint8), bitorder="little")
+        dump_outputs(args.dump_outputs, outputs)
     clocks = sampler.stop() if rank == 0 else None
     value = world * BATCH * args.steps / (dev_ms * 1e-3)
 
